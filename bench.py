@@ -71,6 +71,10 @@ def parse_args():
                          "numbers under the key 'replicas'")
     ap.add_argument("--merge", default="p2p", choices=["p2p", "nccl"],
                     help="shards: hits stored into the owner's buffer over NVLink (p2p) or ids all-reduced (nccl)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="replicas layout: after the timed steps, write what the last timed step returned (calls, window "
+                         "counts, hit lists of a seeded sample of reads) and the run's per-taxon counters as DIR/<name>.npy, "
+                         "so that two builds can be compared output for output")
     return ap.parse_args()
 
 
@@ -270,6 +274,8 @@ def main():
         dist = dist_mod
         dist.init_process_group("nccl", device_id=torch.device(dev))
     mode = resolve_mode(args, world if args.impl == "ours" else 1)
+    if args.dump_outputs and (args.impl != "ours" or mode != "replicas"):
+        raise SystemExit("--dump-outputs writes the outputs of our replicas layout (--impl ours, one GPU or --mode replicas)")
     B = args.batch_reads
     steps_rep = (args.warmup + args.steps) + 5 + (max(args.warmup, 3) + args.steps)
 
@@ -355,6 +361,39 @@ def measure_cpu_baseline(args, w, rank):
                             "sample": f"failed: {e}"[:300]}
 
     return cpu_baseline
+
+
+DUMP_READS = 1 << 20          # per-read outputs of every read of the step, or of a seeded sample of this many
+DUMP_HIT_READS = 1 << 16      # hit lists of a seeded sample of this many of those reads
+
+
+def dump_outputs(out_dir, clf, n_reads, offsets):
+    """What the caller of the timed path receives from its last step — per-read calls (taxids), window counts and
+    run-length hit lists of the batch in slot 0 (kuq_collect_device_batch) — and the per-taxon counters of the run
+    (kuq_read_counts), as float64 / float32 .npy files in out_dir, 64 MB at most."""
+    from krakenuniq_b200 import binding
+    res = binding.BatchResult()
+    clf._ck(clf.L.kuq_collect_device_batch(clf.h, 0, ctypes.byref(res)))
+    r = clf._result(res, offsets)
+    rng = np.random.default_rng(0)
+    reads = np.arange(n_reads) if n_reads <= DUMP_READS else np.sort(rng.choice(n_reads, DUMP_READS, replace=False))
+    hit_reads = np.sort(rng.choice(reads, min(len(reads), DUMP_HIT_READS), replace=False))
+    start = r["run_start"][hit_reads].astype(np.int64)
+    count = r["run_count"][hit_reads].astype(np.int64)
+    runs = np.repeat(start - (np.cumsum(count) - count), count) + np.arange(int(count.sum()))
+    cnt = clf.counts()
+    arrays = {"read_index": reads.astype(np.float64), "call": r["call"][reads].astype(np.float64),
+              "n_windows": r["n_windows"][reads].astype(np.float32),
+              "hit_read_index": hit_reads.astype(np.float64), "hit_run_count": count.astype(np.float64),
+              # one row per run: (taxid, or 0xFFFFFFFF for ambiguous windows; number of windows)
+              "hit_runs": r["runs"][runs].astype(np.float64)}
+    arrays.update({f"taxon_{k}": cnt[k].astype(np.float64) for k in ("taxid", "n_reads", "n_kmers", "unique")})
+    total = sum(a.nbytes for a in arrays.values())
+    if total > 64 << 20:
+        raise RuntimeError(f"--dump-outputs: {total} bytes exceed the 64 MB budget")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def run_replicas(args, w, rank, world, local_rank, dev, dist, cpu_baseline):
@@ -446,6 +485,8 @@ def run_replicas(args, w, rank, world, local_rank, dev, dist, cpu_baseline):
     clf.sync(0)
     barrier()
     harvest_ms_value = clf.sparse_tier_info()["last_harvest_ms"]
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, clf, B, host_offsets)
     sampler.mark(t0, time.time())
     launches = clf.launch_count() - launches0
     dev_ms = ev0.elapsed_time(ev1)

@@ -16,11 +16,3 @@ def pytest_configure(config):
 def oracle():
     from oracle.oracle_py import Oracle
     return Oracle()
-
-
-@pytest.fixture(scope="session")
-def refshim():
-    from oracle import oracle_py
-    if not oracle_py.have_reference():
-        pytest.skip("oracle/_ref not built (needs /root/reference; prebuilt files travel to the GPU box)")
-    return oracle_py.RefShim()

@@ -1,6 +1,8 @@
 """BASELINE configs[1] through the drop-in executable: 8 GB synthetic KrakenDB (666 M records, k=31, m=15), reads of
-the bench workload, our `classify` against the UNMODIFIED reference (`oracle/_ref/classify -M`) — Kraken lines equal
-(as sorted multisets: the reference runs multi-threaded, SURVEY §8(c)) and every report row equal, `kmers` included.
+the bench workload, our `classify` against the UNMODIFIED reference (`classify -M`) — Kraken lines equal (as sorted
+multisets: the reference runs multi-threaded, SURVEY §8(c)) and every report row equal, `kmers` included.  The
+reference's outputs on this seeded workload are pinned by their sha256 in tests/golden/reference/configs1_cli.json
+(written by tests/golden/make_golden_configs1.py on a GPU machine: the database is generated on the device).
 Also times the whole command on a larger FASTQ (tmpfs → Kraken file + report, the reference's own stats-line
 convention) and leaves the numbers in gpurun_out/cli_speed.json for bench.py / DESIGN.md."""
 import json
@@ -17,7 +19,7 @@ from tests import util
 
 pytestmark = pytest.mark.gpu
 
-N_PARITY = int(os.environ.get("KUQ_LARGE_PARITY_READS", 250_000))
+N_PARITY = 250_000                       # the reads the golden digests were taken on
 N_SPEED = int(os.environ.get("KUQ_LARGE_SPEED_READS", 8_000_000))
 
 
@@ -31,16 +33,20 @@ def _rows(path):
     return rows
 
 
-@pytest.fixture(scope="module")
-def workload():
+def kraken_digest(path):
+    """sha256 of the Kraken lines as a sorted multiset"""
+    return util.digest(b"\n".join(sorted(open(path, "rb").read().splitlines())))
+
+
+def report_digest(rows):
+    return util.digest(json.dumps(sorted(rows.items())))
+
+
+def make_workload():
+    """database files, taxDB and the parity / speed FASTQs of the bench workload in tmpfs: (dir, parity fq, speed fq)"""
     import torch
     import bench
     from krakenuniq_b200 import synth_gpu
-    if not os.path.exists(os.path.join(util.ROOT, "oracle", "_ref", "classify")):
-        pytest.skip("oracle/_ref not built")
-    free = os.statvfs("/dev/shm")
-    if free.f_bavail * free.f_frsize < 24 << 30:
-        pytest.skip("needs 24 GB of tmpfs for the database files")
 
     class A:
         cache_dir, db_records, genomes, cpu_sample_reads = "/dev/shm", 666_000_000, 2000, N_PARITY
@@ -57,25 +63,28 @@ def workload():
     return d, fq_par, fq_speed
 
 
+@pytest.fixture(scope="module")
+def workload():
+    free = os.statvfs("/dev/shm")
+    if free.f_bavail * free.f_frsize < 24 << 30:
+        pytest.skip("needs 24 GB of tmpfs for the database files")
+    return make_workload()
+
+
 def test_configs1_cli_parity_with_the_reference(workload, tmp_path):
     d, fq_par, _ = workload
     dbargs = ["-d", f"{d}/database.kdb", "-i", f"{d}/database.idx", "-a", f"{d}/taxDB"]
     threads = str(min(16, os.cpu_count() or 1))
-    r = subprocess.run([os.path.join(util.ROOT, "oracle/_ref/classify")] + dbargs + ["-M", "-t", threads, "-o", str(tmp_path / "ref.kraken"),
-                       "-r", str(tmp_path / "ref.report"), fq_par], capture_output=True, text=True,
-                       env=dict(os.environ, OMP_NUM_THREADS=threads))
-    assert r.returncode == 0, r.stderr[-1000:]
     exe = build.build_classify()
     r2 = subprocess.run([exe] + dbargs + ["-M", "-t", threads, "-o", str(tmp_path / "our.kraken"), "-r", str(tmp_path / "our.report"), fq_par],
                         capture_output=True, text=True, env=dict(os.environ, KUQ_SPARSE_SLOTS=str(1 << 28)))
     assert r2.returncode == 0, r2.stderr[-1500:]
-    ref = sorted(open(tmp_path / "ref.kraken", "rb").read().splitlines())
-    our = sorted(open(tmp_path / "our.kraken", "rb").read().splitlines())
-    assert len(ref) == N_PARITY and ref == our
-    a, b = _rows(tmp_path / "ref.report"), _rows(tmp_path / "our.report")
-    assert len(a) > 2000                                       # 2000 species + genera + families + root + unclassified
-    diff = [k for k in a if a[k] != b.get(k)] + [k for k in b if k not in a]
-    assert not diff, (diff[:5], [a.get(k) for k in diff[:3]], [b.get(k) for k in diff[:3]])
+    ref = util.reference_json("configs1_cli.json")
+    assert ref["reads"] == N_PARITY and ref["report_rows"] > 2000     # 2000 species + genera + families + root + unclassified
+    assert len(open(tmp_path / "our.kraken", "rb").read().splitlines()) == N_PARITY
+    assert kraken_digest(tmp_path / "our.kraken") == ref["kraken_sorted_sha256"]
+    b = _rows(tmp_path / "our.report")
+    assert len(b) == ref["report_rows"] and report_digest(b) == ref["report_rows_sha256"]
 
 
 def test_configs1_cli_throughput(workload, tmp_path):

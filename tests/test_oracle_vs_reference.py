@@ -1,12 +1,27 @@
-"""Pin the C restatement (oracle/kuq_oracle.c) against the UNMODIFIED reference classes (oracle/_ref/libkuref.so),
-function by function, plus the known answers SURVEY.md §8(c) extracted from the compiled reference."""
+"""Pin the C restatement (oracle/kuq_oracle.c) against the UNMODIFIED reference classes, function by function, plus the
+known answers SURVEY.md §8(c) extracted from the compiled reference.  The reference's answers on these seeded inputs
+(oracle/_ref/libkuref.so) are stored in tests/golden/reference/functions.npz by tests/golden/make_golden_reference.py;
+outputs too large to store are pinned by their sha256."""
+import os
+
 import numpy as np
 import pytest
 
 from krakenuniq_b200 import synth
-from oracle.oracle_py import RefHLL
+from tests import util
 
 K = 31
+FMIX_KATS = {0: 0xb456bcfc34c2cb2c, 1: 0x3abf2a20650683e7, 2: 0x0b5181c509f8d8ce,
+             0x0123456789abcdef: 0x6573ed81fcdd91d5, (1 << 62) - 1: 0x6554a70955a989a0}
+BITS_CASES = [(2, 8), (1, 6), (2, 11)]
+# SURVEY §8(c) known answers of the compiled reference: n items → cardinality, default sketch / forced dense p=12
+HLL_KATS = [(1000, 1000), (1024, 1024), (1025, 1017), (2000, 2000), (10000, 9965), (100000, 100000)]
+HLL_DENSE12_KATS = [(1000, 994), (1024, 1015)]
+
+
+@pytest.fixture(scope="module")
+def ref():
+    return np.load(os.path.join(util.REFERENCE, "functions.npz"))
 
 
 def _mini_db(rng, nt=8, idx_type=2, n_genomes=4, glen=1500):
@@ -18,15 +33,16 @@ def _mini_db(rng, nt=8, idx_type=2, n_genomes=4, glen=1500):
     return tax, genomes, km, tx, kdb, idx
 
 
-def test_fmix_kats(oracle, refshim):
-    kats = {0: 0xb456bcfc34c2cb2c, 1: 0x3abf2a20650683e7, 2: 0x0b5181c509f8d8ce,
-            0x0123456789abcdef: 0x6573ed81fcdd91d5, (1 << 62) - 1: 0x6554a70955a989a0}
-    for x, h in kats.items():
+def fmix_inputs():
+    return np.random.default_rng(1).integers(0, 1 << 63, 2000, dtype=np.uint64)
+
+
+def test_fmix_kats(oracle, ref):
+    for x, h in FMIX_KATS.items():
         assert oracle.fmix64(x) == h
-        assert refshim.L.kuref_murmur_fmix(x) == h
-    rng = np.random.default_rng(1)
-    for x in rng.integers(0, 1 << 63, 2000, dtype=np.uint64).tolist():
-        assert oracle.fmix64(x) == refshim.L.kuref_murmur_fmix(x)
+    assert ref["fmix_kats"].tolist() == list(FMIX_KATS.values())
+    got = np.array([oracle.fmix64(x) for x in fmix_inputs().tolist()], np.uint64)
+    assert np.array_equal(got, ref["fmix"])
 
 
 def test_kmer_kat_from_survey(oracle):
@@ -40,49 +56,67 @@ def test_kmer_kat_from_survey(oracle):
     assert oracle.bin_key(canon, K, 8, 2) == 1713
 
 
-@pytest.mark.parametrize("idx_type,nt", [(2, 8), (1, 6), (2, 11)])
-def test_bits_and_lookup_match_reference(oracle, refshim, idx_type, nt):
+def bits_inputs(idx_type, nt):
     rng = np.random.default_rng(10 + nt)
     tax, genomes, km, tx, kdb, idx = _mini_db(rng, nt, idx_type)
-    odb = oracle.open_db(kdb, idx)
-    rdb = refshim.open_db(kdb, idx)
-    assert odb.k == refshim.L.kuref_db_k(rdb.h) == K
-    assert odb.nt == refshim.L.kuref_db_index_nt(rdb.h) == nt
-    assert odb.idx_type == refshim.L.kuref_db_index_type(rdb.h) == idx_type
     probe = np.concatenate([km[rng.integers(0, len(km), 1500)],
                             synth.canonical(rng.integers(0, 1 << 62, 1500, dtype=np.uint64), K)])
-    for x in probe.tolist():
-        assert oracle.canonical(x, K) == rdb.canonical(x)
-        assert oracle.revcomp(x, K) == rdb.revcomp(x, K)
-        assert oracle.revcomp(x & ((1 << 30) - 1), 15) == rdb.revcomp(x & ((1 << 30) - 1), 15)
-        assert oracle.bin_key(x, K, nt, idx_type) == rdb.bin_key(x)
-        assert oracle.bin_key(x, K, nt, 2) == rdb.bin_key_nt(x, nt)
-        assert odb.query(x) == rdb.query(x)
+    return rng, km, tx, kdb, idx, probe
+
+
+def bits_outputs(canonical, revcomp, bin_key, bin_key_nt, query, probe):
+    """The per-probe answers of one implementation, as the arrays whose sha256 the golden file holds."""
+    xs = probe.tolist()
+    low = [x & ((1 << 30) - 1) for x in xs]
+    return {"canonical": np.array([canonical(x) for x in xs], np.uint64),
+            "revcomp": np.array([revcomp(x, K) for x in xs], np.uint64),
+            "revcomp15": np.array([revcomp(x, 15) for x in low], np.uint64),
+            "bin_key": np.array([bin_key(x) for x in xs], np.uint64),
+            "bin_key_nt": np.array([bin_key_nt(x) for x in xs], np.uint64),
+            "query": np.array([query(x) for x in xs], np.uint64)}
+
+
+@pytest.mark.parametrize("idx_type,nt", BITS_CASES)
+def test_bits_and_lookup_match_reference(oracle, ref, idx_type, nt):
+    rng, km, tx, kdb, idx, probe = bits_inputs(idx_type, nt)
+    odb = oracle.open_db(kdb, idx)
+    key = f"bits_{idx_type}_{nt}"
+    assert ref[key + "_header"].tolist() == [K, nt, idx_type]
+    assert [odb.k, odb.nt, odb.idx_type] == [K, nt, idx_type]
+    got = bits_outputs(lambda x: oracle.canonical(x, K), oracle.revcomp, lambda x: oracle.bin_key(x, K, nt, idx_type),
+                       lambda x: oracle.bin_key(x, K, nt, 2), odb.query, probe)
+    for name, arr in got.items():
+        assert util.digest(arr) == str(ref[f"{key}_{name}"]), name
     # numpy generator agrees too (it builds the fixtures)
-    assert np.array_equal(synth.bin_key(probe, K, nt, idx_type),
-                          np.array([rdb.bin_key(x) for x in probe.tolist()], np.uint64))
+    assert util.digest(synth.bin_key(probe, K, nt, idx_type).astype(np.uint64)) == str(ref[key + "_bin_key"])
     # every stored key is found with its taxon; stateful (cached-range) lookups agree with stateless ones
     sel = rng.integers(0, len(km), 500)
     for x, t in zip(km[sel].tolist(), tx[sel].tolist()):
         assert odb.query(x) == (True, t)
 
 
-def test_stateful_query_equals_stateless(oracle, refshim):
+def stateful_inputs(oracle):
+    """canonical k-mers of 200 reads, one array per read"""
     rng = np.random.default_rng(3)
     tax, genomes, km, tx, kdb, idx = _mini_db(rng, 8, 2)
-    odb = oracle.open_db(kdb, idx)
-    rdb = refshim.open_db(kdb, idx)
     reads, offs = synth.sample_reads(rng, genomes, 200, 150, 0.02, 0.0, 0.3)
+    per_read = []
     for i in range(200):
-        seq = reads[int(offs[i]):int(offs[i + 1])].tobytes()
-        kmers, amb = oracle.scan(seq, K)
-        canon = synth.canonical(kmers[amb == 0], K)
-        got = rdb.query_stateful(canon)
-        want = np.array([odb.query(x)[1] for x in canon.tolist()], np.uint32)
-        assert np.array_equal(got, want)
+        kmers, amb = oracle.scan(reads[int(offs[i]):int(offs[i + 1])].tobytes(), K)
+        per_read.append(synth.canonical(kmers[amb == 0], K))
+    return kdb, idx, per_read
 
 
-def test_scanner_matches_reference(oracle, refshim):
+def test_stateful_query_equals_stateless(oracle, ref):
+    """the reference's stateful (cached-range) lookups over each read's k-mers equal the oracle's stateless ones"""
+    kdb, idx, per_read = stateful_inputs(oracle)
+    odb = oracle.open_db(kdb, idx)
+    want = np.split(ref["stateful"], np.cumsum([len(c) for c in per_read])[:-1])
+    for canon, w in zip(per_read, want):
+        assert np.array_equal(np.array([odb.query(x)[1] for x in canon.tolist()], np.uint32), w)
+
+
+def scanner_cases():
     rng = np.random.default_rng(5)
     cases = [b"", b"ACGT", b"A" * 30, b"A" * 31, b"ACGTN" * 20, b"acgtacgtacgtacgtacgtacgtacgtacgtacgt",
              b"ACGT" * 10 + b"\r", b"ACGTAC" * 10 + b"\r", b"ACGTACGTAC" * 6 + b"\r" + b"GATTACA" * 8 + b"\r",
@@ -91,12 +125,19 @@ def test_scanner_matches_reference(oracle, refshim):
         n = int(rng.integers(0, 200))
         alphabet = np.frombuffer(b"ACGTACGTACGTacgtNnRY", np.uint8)
         cases.append(alphabet[rng.integers(0, len(alphabet), n)].tobytes())
-    for seq in cases:
-        k1, a1 = oracle.scan(seq, K)
-        k2, a2 = refshim.scan(seq, K)
-        assert len(k1) == len(k2), seq
-        assert np.array_equal(a1, a2), seq
-        assert np.array_equal(k1[a1 == 0], k2[a2 == 0]), seq
+    return cases
+
+
+def scan_digest(kmers, amb):
+    """window count, ambiguity flags and the k-mers of the unambiguous windows (the others are unspecified)"""
+    return util.digest(np.array([len(kmers)], np.uint64), amb.astype(np.uint8), kmers[amb == 0].astype(np.uint64))
+
+
+def test_scanner_matches_reference(oracle, ref):
+    cases = scanner_cases()
+    assert len(ref["scan"]) == len(cases)
+    for seq, want in zip(cases, ref["scan"]):
+        assert scan_digest(*oracle.scan(seq, K)) == str(want), seq
 
 
 def _random_forest(rng, n, with_one=True):
@@ -118,61 +159,74 @@ def _random_forest(rng, n, with_one=True):
     return ids, parent
 
 
-@pytest.mark.parametrize("with_one", [True, False])
-def test_lca_and_resolve_tree_match_reference(oracle, refshim, with_one):
+def lca_inputs(with_one):
+    """a random forest, 3000 taxon pairs and 1500 hit maps"""
     rng = np.random.default_rng(7 + with_one)
     ids, parent = _random_forest(rng, 300, with_one)
-    opm = oracle.parent_map(ids, parent)
-    rpm = refshim.parent_map(ids, parent)
     pool = np.concatenate([ids, [0, 1, 99999]]).astype(np.uint32)
-    for _ in range(3000):
-        a, b = (int(x) for x in pool[rng.integers(0, len(pool), 2)])
-        assert opm.lca(a, b) == rpm.lca(a, b), (a, b)
+    pairs = [tuple(int(x) for x in pool[rng.integers(0, len(pool), 2)]) for _ in range(3000)]
+    hit_maps = []
     for _ in range(1500):
         n = int(rng.integers(0, 7))
         nz = pool[pool != 0]
         taxa = np.unique(nz[rng.integers(0, len(nz), n)]) if n else np.zeros(0, np.uint32)
-        hits = {int(t): int(rng.integers(1, 4)) for t in taxa}
-        assert opm.resolve_tree(hits) == rpm.resolve_tree(hits), hits
+        hit_maps.append({int(t): int(rng.integers(1, 4)) for t in taxa})
+    return ids, parent, pairs, hit_maps
 
 
-def test_hll_kats_and_state_machine(oracle, refshim):
-    def seq(n, mul=0x9E3779B97F4A7C15, off=0):
-        return ((np.arange(off, off + n, dtype=np.uint64)) * np.uint64(mul))
-    # SURVEY §8(c) known answers of the compiled reference
-    for n, want in [(1000, 1000), (1024, 1024), (1025, 1017), (2000, 2000), (10000, 9965), (100000, 100000)]:
-        o = oracle.hll(); o.insert(seq(n))
-        r = RefHLL(refshim); r.insert(seq(n))
-        assert r.cardinality() == want
+@pytest.mark.parametrize("with_one", [True, False])
+def test_lca_and_resolve_tree_match_reference(oracle, ref, with_one):
+    ids, parent, pairs, hit_maps = lca_inputs(with_one)
+    opm = oracle.parent_map(ids, parent)
+    for (a, b), want in zip(pairs, ref[f"lca_{int(with_one)}"].tolist()):
+        assert opm.lca(a, b) == want, (a, b)
+    for hits, want in zip(hit_maps, ref[f"resolve_{int(with_one)}"].tolist()):
+        assert opm.resolve_tree(hits) == want, hits
+
+
+def hll_seq(n, mul=0x9E3779B97F4A7C15, off=0):
+    return ((np.arange(off, off + n, dtype=np.uint64)) * np.uint64(mul))
+
+
+def test_hll_kats_and_state_machine(oracle, ref):
+    for (n, want), (r_card, r_obs) in zip(HLL_KATS, ref["hll_kats"].tolist()):
+        o = oracle.hll(); o.insert(hll_seq(n))
+        assert r_card == want
         assert o.cardinality() == want
-        assert o.n_observed() == r.n_observed() == n
+        assert o.n_observed() == r_obs == n
         assert o.is_sparse() == (n <= 1024)
     # forced dense p=12 via the registers-only estimator
-    for n, want in [(1000, 994), (1024, 1015)]:
-        r = RefHLL(refshim, dense_p=12); r.insert(seq(n))
-        assert r.cardinality() == want
-        o = oracle.hll(); o.insert(seq(n))
+    for (n, want), r_card in zip(HLL_DENSE12_KATS, ref["hll_dense12"].tolist()):
+        assert r_card == want
+        o = oracle.hll(); o.insert(hll_seq(n))
         assert oracle.ertl_dense(o.registers(), n) == want
     # ten sparse sketches of 1000 merged stay sparse and near exact
-    og, rg = oracle.hll(), RefHLL(refshim)
+    og = oracle.hll()
     for i in range(10):
-        o = oracle.hll(); o.insert(seq(1000, off=1000 * i)); og.merge(o)
-        r = RefHLL(refshim); r.insert(seq(1000, off=1000 * i)); rg.merge(r, move=bool(i & 1))
-    assert og.is_sparse() and og.cardinality() == rg.cardinality() == 10000
+        o = oracle.hll(); o.insert(hll_seq(1000, off=1000 * i)); og.merge(o)
+    assert og.is_sparse() and og.cardinality() == int(ref["hll_merged10"]) == 10000
 
 
-def test_hll_random_merge_sequences(oracle, refshim):
+def hll_merge_sequences():
+    """12 trials of (items, merge by move) parts, duplicates on purpose: items are drawn from a pool about as large as n"""
     rng = np.random.default_rng(11)
+    trials = []
     for trial in range(12):
-        og, rg = oracle.hll(), RefHLL(refshim)
+        parts = []
         for part in range(int(rng.integers(1, 8))):
             n = int(rng.choice([0, 3, 200, 1023, 1024, 1025, 1500, 5000]))
-            # duplicates on purpose: draw from a pool about as large as n
-            items = rng.integers(0, max(n, 1) * int(rng.choice([1, 4, 1000])), n, dtype=np.uint64)
+            parts.append((rng.integers(0, max(n, 1) * int(rng.choice([1, 4, 1000])), n, dtype=np.uint64), bool(part & 1)))
+        trials.append(parts)
+    return trials
+
+
+def test_hll_random_merge_sequences(oracle, ref):
+    """per part: (cardinality of the part, cardinality and items observed of the running merge)"""
+    got = []
+    for parts in hll_merge_sequences():
+        og = oracle.hll()
+        for items, _ in parts:
             o = oracle.hll(); o.insert(items)
-            r = RefHLL(refshim); r.insert(items)
-            assert o.cardinality() == r.cardinality()
             og.merge(o)
-            rg.merge(r, move=bool(part & 1))
-            assert og.cardinality() == rg.cardinality(), (trial, part)
-            assert og.n_observed() == rg.n_observed()
+            got.append((o.cardinality(), og.cardinality(), og.n_observed()))
+    assert np.array_equal(np.array(got, np.uint64), ref["hll_merge"])

@@ -1,12 +1,11 @@
 """The torch workload generator (krakenuniq_b200/synth_gpu.py) writes the reference's on-disk layout: checked on
-CPU tensors against the numpy generator and, where oracle/_ref exists, byte-for-byte against the reference's own
-db_sort."""
-import os
-
+CPU tensors against the numpy generator and byte-for-byte against what the reference's own db_sort made of the same
+records (its sha256 in tests/golden/reference/dbtools.json, written by tests/golden/make_golden_reference.py)."""
 import numpy as np
 import pytest
 
 from krakenuniq_b200 import synth, synth_gpu
+from tests import util
 
 
 def _small(device="cpu", nt=7, idx_type=2):
@@ -32,22 +31,21 @@ def test_layout_matches_numpy_generator(nt, idx_type):
         assert t == db.species[pos[kk] // db.genome_len]
 
 
-def test_matches_reference_db_sort(tmp_path):
-    from oracle import oracle_py
-    if not oracle_py.have_reference():
-        pytest.skip("oracle/_ref not built")
-    db = _small()
-    kdb, idx = db.images()
+def shuffled_records(kdb):
+    """the records of a database image in a seeded random order, as db_sort's unsorted input"""
     k, keys, taxa = synth.parse_kdb(kdb)
-    rng = np.random.default_rng(1)
-    perm = rng.permutation(len(keys))
+    perm = np.random.default_rng(1).permutation(len(keys))
     rec = np.zeros(len(keys), synth._REC)
     rec["key"], rec["taxon"] = keys[perm], taxa[perm]
-    np.concatenate([synth.kdb_header(31, len(keys)), rec.view(np.uint8)]).tofile(tmp_path / "in.jdb")
-    r = oracle_py.run_ref_tool("db_sort", ["-n", 7, "-d", "in.jdb", "-o", "out.kdb", "-i", "out.idx"], cwd=tmp_path)
-    assert r.returncode == 0, r.stderr
-    assert np.array_equal(np.fromfile(tmp_path / "out.kdb", np.uint8), kdb)
-    assert np.array_equal(np.fromfile(tmp_path / "out.idx", np.uint8), idx)
+    return np.concatenate([synth.kdb_header(31, len(keys)), rec.view(np.uint8)])
+
+
+def test_matches_reference_db_sort():
+    """the reference's `db_sort -n 7` of the generator's records, shuffled, gives back the generator's images"""
+    kdb, idx = _small().images()
+    want = util.reference_json("dbtools.json")["synth_gpu_db_sort"]
+    assert util.digest(kdb) == want["kdb"]
+    assert util.digest(idx) == want["idx"]
 
 
 def test_reads_shape_and_content():

@@ -1,11 +1,32 @@
 """Shared helpers for the parity tests (host-side only; no product logic)."""
+import hashlib
+import json
 import os
 
 import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 GOLDEN = os.path.join(ROOT, "tests", "golden", "mini")
+# answers of the unmodified reference on the tests' seeded inputs (tests/golden/make_golden_reference.py)
+REFERENCE = os.path.join(ROOT, "tests", "golden", "reference")
 AMBIG = 0xFFFFFFFF
+
+
+def digest(*parts):
+    """sha256 over arrays / bytes / str in order: pins a reference output too large to store in full."""
+    h = hashlib.sha256()
+    for p in parts:
+        if isinstance(p, str):
+            p = p.encode()
+        elif isinstance(p, np.ndarray):
+            p = np.ascontiguousarray(p).tobytes()
+        h.update(p)
+    return h.hexdigest()
+
+
+def reference_json(name):
+    with open(os.path.join(REFERENCE, name)) as f:
+        return json.load(f)
 
 
 def read_fasta(path):
