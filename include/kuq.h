@@ -179,7 +179,8 @@ int kuq_set_taxonomy(kuq_ctx *ctx, const uint32_t *taxid, const uint32_t *parent
 /* bases: concatenated sequences exactly as DNASequence::seq holds them (seqreader.hpp:27-32), read r =
  * bases[read_offsets[r] .. read_offsets[r+1]).  unit_id: work-unit id per read for the HLL mode rule, or NULL to
  * let the library cut units like process_file does (classify.cpp:514-520, continuing across batches).
- * kuq_classify_batch = submit + wait on slot 0. */
+ * kuq_classify_batch = submit + wait on slot 0.  A slot with an unread batch (kuq_submit_batch without its
+ * kuq_wait_batch yet) refuses every batch call, host or device inputs, with KUQ_E_STATE until kuq_wait_batch. */
 int kuq_classify_batch(kuq_ctx *ctx, const char *bases, const uint64_t *read_offsets, uint32_t n_reads,
                        const uint32_t *unit_id, uint32_t flags, kuq_batch_result *out);
 int kuq_submit_batch(kuq_ctx *ctx, uint32_t slot, const char *bases, const uint64_t *read_offsets,

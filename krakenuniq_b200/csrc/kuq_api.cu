@@ -31,7 +31,6 @@ constexpr uint32_t USET_CAP = 1u << 22;                       // distinct (pair,
 struct Slot {
   cudaStream_t stream = nullptr;
   cudaEvent_t ev_k0 = nullptr, ev_k1 = nullptr, ev_stage[2] = {nullptr, nullptr}, ev_sync = nullptr;
-  double stage_ms[3] = {0, 0, 0};
   // device
   char *d_bases = nullptr, *d_clean = nullptr;
   uint64_t *d_offsets = nullptr;
@@ -61,8 +60,6 @@ struct Slot {
   uint32_t n_reads = 0, flags = 0;
   uint64_t total_bases = 0;
   double kernel_ms = 0;
-  bool external = false;   // inputs are caller-owned device buffers
-  const char *x_bases = nullptr;
 };
 
 }  // namespace
@@ -699,10 +696,10 @@ int launch_on_slot(kuq_ctx *ctx, Slot &s, int mode, Params &p) {
   if (ctx->lca_mode) return fail(ctx, KUQ_E_STATE, "this context built a database (kuq_set_lcas_batch): stage it anew to classify");
   ctx->snap_valid = false;
   p.flags |= ctx->extra_flags;
-  if (mode == MODE_LOOKUP && ctx->mark_zero_hits) p.flags |= 16u;
+  if (mode == MODE_LOOKUP && ctx->mark_zero_hits) p.flags |= F_FOUND_ZERO;
   if (ctx->shard_counting && mode != MODE_FUSED && !ctx->mark_zero_hits && !ctx->quick_min &&
       ctx->cfg.hll_mode != KUQ_HLL_EXACT) {
-    p.flags |= 32u;
+    p.flags |= F_SHARD_COUNTING;
     if (mode == MODE_LOOKUP && p.n_reads && ctx->cfg.hll_mode <= KUQ_HLL_CHUNKED) ctx->seen_dirty = true;
   }
   ctx->merged_summary = false;
@@ -712,14 +709,14 @@ int launch_on_slot(kuq_ctx *ctx, Slot &s, int mode, Params &p) {
     p.flags |= KUQ_F_NO_RUNS;
     s.flags |= KUQ_F_NO_RUNS;
   }
-  if (mode == MODE_RESOLVE && !(p.flags & 4u) && ctx->cfg.hll_mode <= KUQ_HLL_CHUNKED && p.n_reads) {
+  if (mode == MODE_RESOLVE && !(p.flags & KUQ_F_NO_COUNTS) && ctx->cfg.hll_mode <= KUQ_HLL_CHUNKED && p.n_reads) {
     int rrc = reserve_direct_inserts(ctx, s.total_bases);
     if (rrc) return rrc;
     // the set may have moved
     p.sparse.slots = ctx->d_sparse_slots;
     p.sparse.mask = ctx->sparse_cap ? ctx->sparse_cap - 1 : 0;
   }
-  const bool units = mode != MODE_LOOKUP && ctx->cfg.hll_mode == KUQ_HLL_PRELOAD && p.unit_id && !(p.flags & 4u);
+  const bool units = mode != MODE_LOOKUP && ctx->cfg.hll_mode == KUQ_HLL_PRELOAD && p.unit_id && !(p.flags & KUQ_F_NO_COUNTS);
   if (units) {
     int rc = prepare_unit_map(ctx, s);
     if (rc) return rc;
@@ -733,13 +730,13 @@ int launch_on_slot(kuq_ctx *ctx, Slot &s, int mode, Params &p) {
   CU(cudaEventRecord(s.ev_stage[1], s.stream));
   if (p.n_reads) ctx->launches += launch_classify(mode, p, ctx->n_sm, s.stream, s.ev_stage);
   // the fused path flags the records of its counted hits (k_lookup); quick / exact runs go through the other halves
-  if (p.n_reads && mode == MODE_FUSED && !(p.flags & 4u) && ctx->cfg.hll_mode <= KUQ_HLL_CHUNKED &&
+  if (p.n_reads && mode == MODE_FUSED && !(p.flags & KUQ_F_NO_COUNTS) && ctx->cfg.hll_mode <= KUQ_HLL_CHUNKED &&
       !(ctx->quick_min && ctx->quick_stop))
     ctx->seen_dirty = true;
   CU(cudaEventRecord(s.ev_k1, s.stream));
   s.timed = true;
   // HLL mode rule: which taxa have a sketch that converted to dense (SURVEY.md App. C)
-  if (p.n_reads && mode != MODE_LOOKUP && !(p.flags & 4u)) {
+  if (p.n_reads && mode != MODE_LOOKUP && !(p.flags & KUQ_F_NO_COUNTS)) {
     if (units) ctx->launches += launch_unit_accounting(p, ctx->n_sm, s.stream);
     else if (ctx->cfg.hll_mode == KUQ_HLL_CHUNKED) {
       launch_flag_dense_global(ctx->d_sparse_distinct, ctx->d_dense_flag, ctx->n_sketch, s.stream);
@@ -1035,15 +1032,34 @@ int kuq_set_taxonomy(kuq_ctx *ctx, const uint32_t *taxid, const uint32_t *parent
 
 // ---- classification -------------------------------------------------------------------------------------------
 namespace {
-// copy one batch of reads (host) into the slot; returns the total number of bases
-int upload_reads(kuq_ctx *ctx, Slot &s, const char *bases, const uint64_t *read_offsets, uint32_t n_reads, uint64_t *total_out) {
+// What every batch call checks before it touches slot `slot`; then the slot records the batch.  A slot with an unread
+// batch refuses every call until kuq_wait_batch: a new launch would overwrite the results it has not copied yet.
+// Device inputs must also be non-NULL and 16-byte aligned (TMA bulk loads); the callers check host inputs.
+int begin_batch(kuq_ctx *ctx, uint32_t slot, uint32_t n_reads, uint64_t total_bases, uint32_t flags, bool device_inputs,
+                const char *d_bases = nullptr, const uint64_t *d_offsets = nullptr) {
+  int rc = check_slot(ctx, slot);
+  if (rc) return rc;
+  if (device_inputs) {
+    if (n_reads && (!d_bases || !d_offsets)) return fail(ctx, KUQ_E_INVALID_ARG, "NULL device buffers");
+    if ((uintptr_t)d_bases & 15) return fail(ctx, KUQ_E_INVALID_ARG, "d_bases must be 16-byte aligned");
+  }
+  CU(cudaSetDevice(ctx->device));
+  Slot &s = ctx->slots[slot];
+  if (s.busy) return fail(ctx, KUQ_E_STATE, "slot %u still has an unread batch: call kuq_wait_batch first", slot);
   if (n_reads > ctx->cfg.max_reads_per_batch) return fail(ctx, KUQ_E_CAPACITY, "%u reads > slot capacity %u", n_reads, ctx->cfg.max_reads_per_batch);
-  const uint64_t base0 = n_reads ? read_offsets[0] : 0;
-  const uint64_t total = n_reads ? read_offsets[n_reads] - base0 : 0;
-  if (total > ctx->cfg.max_bases_per_batch) return fail(ctx, KUQ_E_CAPACITY, "%llu bases > slot capacity %llu", (unsigned long long)total, (unsigned long long)ctx->cfg.max_bases_per_batch);
-  if (total >= (1ull << 32)) return fail(ctx, KUQ_E_CAPACITY, "batches are limited to 4 Gbases");
-  *total_out = total;
+  if (total_bases > ctx->cfg.max_bases_per_batch) return fail(ctx, KUQ_E_CAPACITY, "%llu bases > slot capacity %llu", (unsigned long long)total_bases, (unsigned long long)ctx->cfg.max_bases_per_batch);
+  if (total_bases >= (1ull << 32)) return fail(ctx, KUQ_E_CAPACITY, "batches are limited to 4 Gbases");
+  s.n_reads = n_reads; s.flags = flags; s.total_bases = total_bases;
+  return KUQ_OK;
+}
+
+uint64_t host_bases(const uint64_t *read_offsets, uint32_t n_reads) { return n_reads ? read_offsets[n_reads] - read_offsets[0] : 0; }
+
+// copy the batch begin_batch recorded (reads on the host) into the slot's device buffers
+int upload_reads(kuq_ctx *ctx, Slot &s, const char *bases, const uint64_t *read_offsets) {
+  const uint32_t n_reads = s.n_reads;
   if (!n_reads) return KUQ_OK;
+  const uint64_t base0 = read_offsets[0], total = s.total_bases;
   CU(cudaMemcpyAsync(s.d_bases, bases + base0, total, cudaMemcpyHostToDevice, s.stream));
   CU(cudaMemsetAsync(s.d_bases + total, 'N', SLACK, s.stream));
   if (base0 == 0) {
@@ -1055,30 +1071,88 @@ int upload_reads(kuq_ctx *ctx, Slot &s, const char *bases, const uint64_t *read_
   }
   return KUQ_OK;
 }
+
+// Work-unit id of every read for the KUQ_HLL_PRELOAD rule, on the device: the caller's, or cut like process_file does.
+// *d_unit stays nullptr when the rule needs none.
+int upload_units(kuq_ctx *ctx, Slot &s, const uint64_t *read_offsets, const uint32_t *unit_id, const uint32_t **d_unit) {
+  *d_unit = nullptr;
+  if (ctx->cfg.hll_mode != KUQ_HLL_PRELOAD || !s.n_reads) return KUQ_OK;
+  if (unit_id) memcpy(s.h_unit, unit_id, s.n_reads * 4ull);
+  else cut_units(ctx, read_offsets, s.n_reads, s.h_unit);
+  CU(cudaMemcpyAsync(s.d_unit, s.h_unit, s.n_reads * 4ull, cudaMemcpyHostToDevice, s.stream));
+  *d_unit = s.d_unit;
+  return KUQ_OK;
+}
+
+// Host inputs: begin_batch, a staged database, the reads (and for the counting modes the work-unit ids) copied into the
+// slot, and `p` filled over those copies; the caller adds the fields of `mode` and launches.
+int host_call(kuq_ctx *ctx, uint32_t slot, int mode, const char *bases, const uint64_t *read_offsets, uint32_t n_reads,
+              const uint32_t *unit_id, uint32_t flags, Params &p) {
+  int rc = begin_batch(ctx, slot, n_reads, host_bases(read_offsets, n_reads), flags, false);
+  if (!rc) rc = ensure_ready(ctx);
+  if (rc) return rc;
+  Slot &s = ctx->slots[slot];
+  const uint32_t *d_unit = nullptr;
+  rc = upload_reads(ctx, s, bases, read_offsets);
+  if (!rc && mode != MODE_LOOKUP) rc = upload_units(ctx, s, read_offsets, unit_id, &d_unit);
+  if (rc) return rc;
+  fill_params(ctx, s, p, s.d_bases, s.d_offsets, d_unit, n_reads, flags);
+  return KUQ_OK;
+}
+
+// Device inputs: begin_batch, a staged database, and `p` filled over the caller's buffers; the caller adds the fields of
+// `mode` and launches.
+int device_call(kuq_ctx *ctx, uint32_t slot, int mode, const char *d_bases, const uint64_t *d_offsets, uint32_t n_reads,
+                uint64_t total_bases, const uint32_t *d_unit, uint32_t flags, Params &p) {
+  int rc = begin_batch(ctx, slot, n_reads, total_bases, flags, true, d_bases, d_offsets);
+  if (!rc) rc = ensure_ready(ctx);
+  if (rc) return rc;
+  if (mode != MODE_LOOKUP && ctx->cfg.hll_mode == KUQ_HLL_PRELOAD && !d_unit && !(flags & KUQ_F_NO_COUNTS) && n_reads)
+    return fail(ctx, KUQ_E_INVALID_ARG, "KUQ_HLL_PRELOAD needs the work-unit id of every read (d_unit_id) to "
+                "reproduce the per-unit sketches; pass it, or create the context with KUQ_HLL_CHUNKED / KUQ_HLL_DENSE_ONLY");
+  fill_params(ctx, ctx->slots[slot], p, d_bases, d_offsets, d_unit, n_reads, flags);
+  return KUQ_OK;
+}
+
+// D2H of the batch's fixed-size results into the slot's pinned buffers; the variable-size hit lists follow in
+// kuq_wait_batch, which the slot now waits for
+int copy_results(kuq_ctx *ctx, Slot &s) {
+  if (s.n_reads) {
+    CU(cudaMemcpyAsync(s.h_call, s.d_call, s.n_reads * 4ull, cudaMemcpyDeviceToHost, s.stream));
+    CU(cudaMemcpyAsync(s.h_nwin, s.d_nwin, s.n_reads * 4ull, cudaMemcpyDeviceToHost, s.stream));
+    if (!(s.flags & KUQ_F_NO_RUNS) || ctx->quick_min) {
+      CU(cudaMemcpyAsync(s.h_run_start, s.d_run_start, s.n_reads * 4ull, cudaMemcpyDeviceToHost, s.stream));
+      CU(cudaMemcpyAsync(s.h_run_count, s.d_run_count, s.n_reads * 4ull, cudaMemcpyDeviceToHost, s.stream));
+    }
+  }
+  CU(cudaMemcpyAsync(s.h_scalars, s.d_scalars, 8 * 8, cudaMemcpyDeviceToHost, s.stream));
+  s.busy = true;
+  return KUQ_OK;
+}
+
+// the error word the kernels of the slot's last batch left (Params::error_flag) as a libkuq error code
+int batch_error(kuq_ctx *ctx, const Slot &s, uint32_t err) {
+  if (err == 1) return fail(ctx, KUQ_E_TAXA_OVERFLOW, "the batch exhausted the hit-table pool for reads with more than 32 distinct taxa: use smaller batches");
+  if (err == 4) return fail(ctx, KUQ_E_CAPACITY, "sparse-tier set saturated: raise kuq_config.sparse_set_slots (now %llu)", (unsigned long long)ctx->sparse_cap);
+  if (err == 5) return fail(ctx, KUQ_E_CAPACITY, "the hit lists of the batch need more run slots than the slot holds (%llu): use smaller batches", (unsigned long long)s.runs_cap);
+  if (err) return fail(ctx, KUQ_E_CAPACITY, "per-batch work-unit bookkeeping overflowed (code %u): use smaller batches", err);
+  return KUQ_OK;
+}
 }  // namespace
 
 int kuq_lookup_batch(kuq_ctx *ctx, const char *bases, const uint64_t *read_offsets, uint32_t n_reads,
                      uint32_t *codes_out, uint32_t *n_windows_out) {
-  int rc = check_slot(ctx, 0);
-  if (rc) return rc;
   if (n_reads && (!bases || !read_offsets || !codes_out)) return fail(ctx, KUQ_E_INVALID_ARG, "NULL batch buffers");
-  CU(cudaSetDevice(ctx->device));
-  Slot &s = ctx->slots[0];
-  if (s.busy) return fail(ctx, KUQ_E_STATE, "slot 0 still has an unread batch");
-  rc = ensure_ready(ctx);
-  if (rc) return rc;
-  uint64_t total = 0;
-  rc = upload_reads(ctx, s, bases, read_offsets, n_reads, &total);
-  if (rc) return rc;
-  s.n_reads = n_reads; s.flags = 0; s.total_bases = total; s.external = false;
   Params p;
-  fill_params(ctx, s, p, s.d_bases, s.d_offsets, nullptr, n_reads, 0);
+  int rc = host_call(ctx, 0, MODE_LOOKUP, bases, read_offsets, n_reads, nullptr, 0, p);
+  if (rc) return rc;
+  Slot &s = ctx->slots[0];
   // positions without a window are not written by the kernels: give the caller zeros there
-  CU(cudaMemsetAsync(s.d_dense, 0, total * 4, s.stream));
+  CU(cudaMemsetAsync(s.d_dense, 0, s.total_bases * 4, s.stream));
   rc = launch_on_slot(ctx, s, MODE_LOOKUP, p);
   if (rc) return rc;
   if (n_reads) {
-    CU(cudaMemcpyAsync(codes_out, s.d_dense, total * 4, cudaMemcpyDeviceToHost, s.stream));
+    CU(cudaMemcpyAsync(codes_out, s.d_dense, s.total_bases * 4, cudaMemcpyDeviceToHost, s.stream));
     if (n_windows_out) CU(cudaMemcpyAsync(n_windows_out, s.d_nwin, n_reads * 4ull, cudaMemcpyDeviceToHost, s.stream));
   }
   CU(cudaStreamSynchronize(s.stream));
@@ -1087,82 +1161,25 @@ int kuq_lookup_batch(kuq_ctx *ctx, const char *bases, const uint64_t *read_offse
 
 int kuq_resolve_batch(kuq_ctx *ctx, const char *bases, const uint64_t *read_offsets, uint32_t n_reads,
                       const uint32_t *codes_in, const uint32_t *unit_id, uint32_t flags, kuq_batch_result *out) {
-  int rc = check_slot(ctx, 0);
-  if (rc) return rc;
   if (!out || (n_reads && (!bases || !read_offsets || !codes_in))) return fail(ctx, KUQ_E_INVALID_ARG, "NULL batch buffers");
-  CU(cudaSetDevice(ctx->device));
-  Slot &s = ctx->slots[0];
-  if (s.busy) return fail(ctx, KUQ_E_STATE, "slot 0 still has an unread batch");
-  rc = ensure_ready(ctx);
-  if (rc) return rc;
-  uint64_t total = 0;
-  rc = upload_reads(ctx, s, bases, read_offsets, n_reads, &total);
-  if (rc) return rc;
-  if (!s.d_codes_in) CU(dmalloc(&s.d_codes_in, ctx->cfg.max_bases_per_batch + SLACK));
-  if (n_reads) CU(cudaMemcpyAsync(s.d_codes_in, codes_in, total * 4, cudaMemcpyHostToDevice, s.stream));
-  s.n_reads = n_reads; s.flags = flags; s.total_bases = total; s.external = false;
-  const uint32_t *d_unit = nullptr;
-  if (ctx->cfg.hll_mode == KUQ_HLL_PRELOAD && n_reads) {
-    if (unit_id) memcpy(s.h_unit, unit_id, n_reads * 4ull);
-    else cut_units(ctx, read_offsets, n_reads, s.h_unit);
-    CU(cudaMemcpyAsync(s.d_unit, s.h_unit, n_reads * 4ull, cudaMemcpyHostToDevice, s.stream));
-    d_unit = s.d_unit;
-  }
   Params p;
-  fill_params(ctx, s, p, s.d_bases, s.d_offsets, d_unit, n_reads, flags);
+  int rc = host_call(ctx, 0, MODE_RESOLVE, bases, read_offsets, n_reads, unit_id, flags, p);
+  if (rc) return rc;
+  Slot &s = ctx->slots[0];
+  if (!s.d_codes_in) CU(dmalloc(&s.d_codes_in, ctx->cfg.max_bases_per_batch + SLACK));
+  if (n_reads) CU(cudaMemcpyAsync(s.d_codes_in, codes_in, s.total_bases * 4, cudaMemcpyHostToDevice, s.stream));
   p.codes_in = s.d_codes_in;
   rc = launch_on_slot(ctx, s, MODE_RESOLVE, p);
-  if (rc) return rc;
-  if (n_reads) {
-    CU(cudaMemcpyAsync(s.h_call, s.d_call, n_reads * 4ull, cudaMemcpyDeviceToHost, s.stream));
-    CU(cudaMemcpyAsync(s.h_nwin, s.d_nwin, n_reads * 4ull, cudaMemcpyDeviceToHost, s.stream));
-    if (!(flags & KUQ_F_NO_RUNS) || ctx->quick_min) {
-      CU(cudaMemcpyAsync(s.h_run_start, s.d_run_start, n_reads * 4ull, cudaMemcpyDeviceToHost, s.stream));
-      CU(cudaMemcpyAsync(s.h_run_count, s.d_run_count, n_reads * 4ull, cudaMemcpyDeviceToHost, s.stream));
-    }
-  }
-  CU(cudaMemcpyAsync(s.h_scalars, s.d_scalars, 8 * 8, cudaMemcpyDeviceToHost, s.stream));
-  s.busy = true;
-  return kuq_wait_batch(ctx, 0, out);
+  return rc ? rc : kuq_collect_device_batch(ctx, 0, out);
 }
 
 int kuq_submit_batch(kuq_ctx *ctx, uint32_t slot, const char *bases, const uint64_t *read_offsets, uint32_t n_reads,
                      const uint32_t *unit_id, uint32_t flags) {
-  int rc = check_slot(ctx, slot);
-  if (rc) return rc;
   if (n_reads && (!bases || !read_offsets)) return fail(ctx, KUQ_E_INVALID_ARG, "NULL batch buffers");
-  CU(cudaSetDevice(ctx->device));
-  Slot &s = ctx->slots[slot];
-  if (s.busy) return fail(ctx, KUQ_E_STATE, "slot %u still has an unread batch: call kuq_wait_batch first", slot);
-  rc = ensure_ready(ctx);
-  if (rc) return rc;
-  uint64_t total = 0;
-  rc = upload_reads(ctx, s, bases, read_offsets, n_reads, &total);
-  if (rc) return rc;
-  s.n_reads = n_reads; s.flags = flags; s.total_bases = total; s.external = false;
-  const uint32_t *d_unit = nullptr;
-  if (ctx->cfg.hll_mode == KUQ_HLL_PRELOAD && n_reads) {
-    if (unit_id) memcpy(s.h_unit, unit_id, n_reads * 4ull);
-    else cut_units(ctx, read_offsets, n_reads, s.h_unit);
-    CU(cudaMemcpyAsync(s.d_unit, s.h_unit, n_reads * 4ull, cudaMemcpyHostToDevice, s.stream));
-    d_unit = s.d_unit;
-  }
   Params p;
-  fill_params(ctx, s, p, s.d_bases, s.d_offsets, d_unit, n_reads, flags);
-  rc = launch_on_slot(ctx, s, MODE_FUSED, p);
-  if (rc) return rc;
-  // D2H of the fixed-size results; the variable-size hit lists follow in kuq_wait_batch
-  if (n_reads) {
-    CU(cudaMemcpyAsync(s.h_call, s.d_call, n_reads * 4ull, cudaMemcpyDeviceToHost, s.stream));
-    CU(cudaMemcpyAsync(s.h_nwin, s.d_nwin, n_reads * 4ull, cudaMemcpyDeviceToHost, s.stream));
-    if (!(flags & KUQ_F_NO_RUNS) || ctx->quick_min) {
-      CU(cudaMemcpyAsync(s.h_run_start, s.d_run_start, n_reads * 4ull, cudaMemcpyDeviceToHost, s.stream));
-      CU(cudaMemcpyAsync(s.h_run_count, s.d_run_count, n_reads * 4ull, cudaMemcpyDeviceToHost, s.stream));
-    }
-  }
-  CU(cudaMemcpyAsync(s.h_scalars, s.d_scalars, 8 * 8, cudaMemcpyDeviceToHost, s.stream));
-  s.busy = true;
-  return KUQ_OK;
+  int rc = host_call(ctx, slot, MODE_FUSED, bases, read_offsets, n_reads, unit_id, flags, p);
+  if (!rc) rc = launch_on_slot(ctx, ctx->slots[slot], MODE_FUSED, p);
+  return rc ? rc : copy_results(ctx, ctx->slots[slot]);
 }
 
 int kuq_wait_batch(kuq_ctx *ctx, uint32_t slot, kuq_batch_result *out) {
@@ -1178,11 +1195,8 @@ int kuq_wait_batch(kuq_ctx *ctx, uint32_t slot, kuq_batch_result *out) {
   if (s.timed) cudaEventElapsedTime(&ms, s.ev_k0, s.ev_k1);
   (void)cudaGetLastError();
   s.kernel_ms = ms;
-  const uint32_t err = (uint32_t)(s.h_scalars[3] & 0xFFFFFFFFu);
-  if (err == 1) return fail(ctx, KUQ_E_TAXA_OVERFLOW, "the batch exhausted the hit-table pool for reads with more than 32 distinct taxa: use smaller batches");
-  if (err == 4) return fail(ctx, KUQ_E_CAPACITY, "sparse-tier set saturated: raise kuq_config.sparse_set_slots (now %llu)", (unsigned long long)ctx->sparse_cap);
-  if (err == 5) return fail(ctx, KUQ_E_CAPACITY, "the hit lists of the batch need more run slots than the slot holds (%llu): use smaller batches", (unsigned long long)s.runs_cap);
-  if (err) return fail(ctx, KUQ_E_CAPACITY, "per-batch work-unit bookkeeping overflowed (code %u): use smaller batches", err);
+  rc = batch_error(ctx, s, (uint32_t)(s.h_scalars[3] & 0xFFFFFFFFu));
+  if (rc) return rc;
   const uint64_t n_runs = (s.flags & KUQ_F_NO_RUNS) ? 0 : s.h_scalars[0];
   if (n_runs) {
     if (n_runs > s.h_runs_cap) {
@@ -1219,68 +1233,45 @@ int kuq_classify_batch(kuq_ctx *ctx, const char *bases, const uint64_t *read_off
   return kuq_wait_batch(ctx, 0, out);
 }
 
-static int device_call(kuq_ctx *ctx, uint32_t slot, int mode, const char *d_bases, const uint64_t *d_offsets,
-                       uint32_t n_reads, uint64_t total_bases, const uint32_t *d_unit, uint32_t flags,
-                       uint32_t *d_codes_out, const uint32_t *d_codes_in, uint32_t only_hits) {
-  int rc = check_slot(ctx, slot);
-  if (rc) return rc;
-  if (n_reads && (!d_bases || !d_offsets)) return fail(ctx, KUQ_E_INVALID_ARG, "NULL device buffers");
-  if ((uintptr_t)d_bases & 15) return fail(ctx, KUQ_E_INVALID_ARG, "d_bases must be 16-byte aligned");
-  CU(cudaSetDevice(ctx->device));
-  rc = ensure_ready(ctx);
-  if (rc) return rc;
-  if (mode != MODE_LOOKUP && ctx->cfg.hll_mode == KUQ_HLL_PRELOAD && !d_unit && !(flags & KUQ_F_NO_COUNTS) && n_reads)
-    return fail(ctx, KUQ_E_INVALID_ARG, "KUQ_HLL_PRELOAD needs the work-unit id of every read (d_unit_id) to "
-                "reproduce the per-unit sketches; pass it, or create the context with KUQ_HLL_CHUNKED / KUQ_HLL_DENSE_ONLY");
-  Slot &s = ctx->slots[slot];
-  if (n_reads > ctx->cfg.max_reads_per_batch || total_bases > ctx->cfg.max_bases_per_batch)
-    return fail(ctx, KUQ_E_CAPACITY, "batch exceeds the slot capacity");
-  s.n_reads = n_reads; s.flags = flags; s.total_bases = total_bases; s.external = true;
-  Params p;
-  fill_params(ctx, s, p, d_bases, d_offsets, d_unit, n_reads, flags);
-  if (mode == MODE_LOOKUP) { p.codes_dense = d_codes_out; p.only_hits = only_hits; }
-  if (mode == MODE_RESOLVE) p.codes_in = d_codes_in;
-  return launch_on_slot(ctx, s, mode, p);
-}
-
 int kuq_classify_device(kuq_ctx *ctx, uint32_t slot, const char *d_bases, const uint64_t *d_read_offsets,
                         uint32_t n_reads, uint64_t total_bases, const uint32_t *d_unit_id, uint32_t flags) {
-  return device_call(ctx, slot, MODE_FUSED, d_bases, d_read_offsets, n_reads, total_bases, d_unit_id, flags, nullptr, nullptr, 0);
+  Params p;
+  int rc = device_call(ctx, slot, MODE_FUSED, d_bases, d_read_offsets, n_reads, total_bases, d_unit_id, flags, p);
+  return rc ? rc : launch_on_slot(ctx, ctx->slots[slot], MODE_FUSED, p);
 }
 int kuq_lookup_device(kuq_ctx *ctx, uint32_t slot, const char *d_bases, const uint64_t *d_read_offsets,
                       uint32_t n_reads, uint64_t total_bases, uint32_t *d_codes_out, uint32_t only_hits) {
   if (!d_codes_out) return KUQ_E_INVALID_ARG;
-  return device_call(ctx, slot, MODE_LOOKUP, d_bases, d_read_offsets, n_reads, total_bases, nullptr, 0, d_codes_out, nullptr, only_hits);
+  Params p;
+  int rc = device_call(ctx, slot, MODE_LOOKUP, d_bases, d_read_offsets, n_reads, total_bases, nullptr, 0, p);
+  if (rc) return rc;
+  p.codes_dense = d_codes_out;
+  p.only_hits = only_hits;
+  return launch_on_slot(ctx, ctx->slots[slot], MODE_LOOKUP, p);
 }
 int kuq_resolve_device(kuq_ctx *ctx, uint32_t slot, const char *d_bases, const uint64_t *d_read_offsets,
                        uint32_t n_reads, uint64_t total_bases, const uint32_t *d_codes_in, const uint32_t *d_unit_id,
                        uint32_t flags) {
   if (!d_codes_in) return KUQ_E_INVALID_ARG;
-  return device_call(ctx, slot, MODE_RESOLVE, d_bases, d_read_offsets, n_reads, total_bases, d_unit_id, flags, nullptr, d_codes_in, 0);
+  Params p;
+  int rc = device_call(ctx, slot, MODE_RESOLVE, d_bases, d_read_offsets, n_reads, total_bases, d_unit_id, flags, p);
+  if (rc) return rc;
+  p.codes_in = d_codes_in;
+  return launch_on_slot(ctx, ctx->slots[slot], MODE_RESOLVE, p);
 }
 
 int kuq_lookup_device_peers(kuq_ctx *ctx, uint32_t slot, const char *d_bases, const uint64_t *d_read_offsets,
                             uint32_t n_reads, uint64_t total_bases, uint32_t *const *d_codes_peers,
                             const uint64_t *base_bounds, uint32_t n_peers) {
   if (!d_codes_peers || !base_bounds || n_peers == 0 || n_peers > 8) return KUQ_E_INVALID_ARG;
-  int rc = check_slot(ctx, slot);
-  if (rc) return rc;
-  if (n_reads && (!d_bases || !d_read_offsets)) return fail(ctx, KUQ_E_INVALID_ARG, "NULL device buffers");
-  if ((uintptr_t)d_bases & 15) return fail(ctx, KUQ_E_INVALID_ARG, "d_bases must be 16-byte aligned");
-  CU(cudaSetDevice(ctx->device));
-  rc = ensure_ready(ctx);
-  if (rc) return rc;
-  Slot &s = ctx->slots[slot];
-  if (n_reads > ctx->cfg.max_reads_per_batch || total_bases > ctx->cfg.max_bases_per_batch)
-    return fail(ctx, KUQ_E_CAPACITY, "batch exceeds the slot capacity");
-  s.n_reads = n_reads; s.flags = 0; s.total_bases = total_bases; s.external = true;
   Params p;
-  fill_params(ctx, s, p, d_bases, d_read_offsets, nullptr, n_reads, 0);
+  int rc = device_call(ctx, slot, MODE_LOOKUP, d_bases, d_read_offsets, n_reads, total_bases, nullptr, 0, p);
+  if (rc) return rc;
   p.only_hits = 1;
   p.n_peers = n_peers;
   for (uint32_t j = 0; j < n_peers; j++) { p.peer_codes[j] = d_codes_peers[j]; p.peer_bounds[j] = base_bounds[j]; }
   p.peer_bounds[n_peers] = base_bounds[n_peers];
-  return launch_on_slot(ctx, s, MODE_LOOKUP, p);
+  return launch_on_slot(ctx, ctx->slots[slot], MODE_LOOKUP, p);
 }
 
 // ---- device memory that can be shared with the other ranks of a node (CUDA IPC) --------------------------------
@@ -1352,18 +1343,8 @@ int kuq_collect_device_batch(kuq_ctx *ctx, uint32_t slot, kuq_batch_result *out)
   CU(cudaSetDevice(ctx->device));
   Slot &s = ctx->slots[slot];
   if (s.busy) return fail(ctx, KUQ_E_STATE, "slot %u still has an unread batch", slot);
-  const uint32_t n_reads = s.n_reads;
-  if (n_reads) {
-    CU(cudaMemcpyAsync(s.h_call, s.d_call, n_reads * 4ull, cudaMemcpyDeviceToHost, s.stream));
-    CU(cudaMemcpyAsync(s.h_nwin, s.d_nwin, n_reads * 4ull, cudaMemcpyDeviceToHost, s.stream));
-    if (!(s.flags & KUQ_F_NO_RUNS) || ctx->quick_min) {
-      CU(cudaMemcpyAsync(s.h_run_start, s.d_run_start, n_reads * 4ull, cudaMemcpyDeviceToHost, s.stream));
-      CU(cudaMemcpyAsync(s.h_run_count, s.d_run_count, n_reads * 4ull, cudaMemcpyDeviceToHost, s.stream));
-    }
-  }
-  CU(cudaMemcpyAsync(s.h_scalars, s.d_scalars, 8 * 8, cudaMemcpyDeviceToHost, s.stream));
-  s.busy = true;
-  return kuq_wait_batch(ctx, slot, out);
+  rc = copy_results(ctx, s);
+  return rc ? rc : kuq_wait_batch(ctx, slot, out);
 }
 
 int kuq_sync_slot(kuq_ctx *ctx, uint32_t slot) {
@@ -1380,11 +1361,7 @@ int kuq_sync_slot(kuq_ctx *ctx, uint32_t slot) {
     if (err) return fail(ctx, KUQ_E_STATE, "kuq_wait_flags timed out: a peer GPU never signalled (code %u)", err);
   }
   CU(cudaMemcpy(&err, reinterpret_cast<uint32_t *>(s.d_scalars + 3), 4, cudaMemcpyDeviceToHost));
-  if (err == 1) return fail(ctx, KUQ_E_TAXA_OVERFLOW, "the batch exhausted the hit-table pool for reads with more than 32 distinct taxa: use smaller batches");
-  if (err == 4) return fail(ctx, KUQ_E_CAPACITY, "sparse-tier set saturated: raise kuq_config.sparse_set_slots (now %llu)", (unsigned long long)ctx->sparse_cap);
-  if (err == 5) return fail(ctx, KUQ_E_CAPACITY, "the hit lists of the batch need more run slots than the slot holds (%llu): use smaller batches", (unsigned long long)s.runs_cap);
-  if (err) return fail(ctx, KUQ_E_CAPACITY, "per-batch work-unit bookkeeping overflowed (code %u): use smaller batches", err);
-  return KUQ_OK;
+  return batch_error(ctx, s, err);
 }
 
 int kuq_slot_device_result(kuq_ctx *ctx, uint32_t slot, kuq_device_result *out) {
@@ -2389,15 +2366,11 @@ uint64_t kuq_ertl_sparse(const uint32_t *hist64, uint64_t n_observed) {
 int kuq_scan_device(kuq_ctx *ctx, uint32_t slot, uint32_t k, uint32_t nt, uint32_t idx_type, const char *d_bases,
                     const uint64_t *d_read_offsets, uint32_t n_reads, uint64_t total_bases, uint64_t *d_canon_out,
                     uint32_t *d_bins_out) {
-  int rc = check_slot(ctx, slot);
-  if (rc) return rc;
   if (!d_bases || !d_read_offsets || !d_canon_out || !d_bins_out) return fail(ctx, KUQ_E_INVALID_ARG, "NULL device buffers");
-  if ((uintptr_t)d_bases & 15) return fail(ctx, KUQ_E_INVALID_ARG, "d_bases must be 16-byte aligned");
   if (k < 2 || k > 31 || nt < 1 || nt > 15 || nt > k || (idx_type != 1 && idx_type != 2)) return fail(ctx, KUQ_E_INVALID_ARG, "bad k / minimizer length / index type");
-  CU(cudaSetDevice(ctx->device));
+  int rc = begin_batch(ctx, slot, n_reads, total_bases, 0, true, d_bases, d_read_offsets);
+  if (rc) return rc;
   Slot &s = ctx->slots[slot];
-  if (n_reads > ctx->cfg.max_reads_per_batch || total_bases > ctx->cfg.max_bases_per_batch)
-    return fail(ctx, KUQ_E_CAPACITY, "batch exceeds the slot capacity");
   Params p;
   memset(&p, 0, sizeof p);
   p.db.k = k; p.db.nt = nt;
@@ -2544,15 +2517,11 @@ int kuq_db_sort(int device, const void *jdb_image, uint64_t jdb_bytes, uint32_t 
 
 int kuq_set_lcas_batch(kuq_ctx *ctx, const char *bases, const uint64_t *piece_offsets, uint32_t n_pieces,
                        const uint32_t *taxid, uint32_t flags, uint64_t *n_missing) {
-  int rc = check_slot(ctx, 0);
-  if (rc) return rc;
   if (n_pieces && (!bases || !piece_offsets || !taxid)) return fail(ctx, KUQ_E_INVALID_ARG, "NULL batch buffers");
-  CU(cudaSetDevice(ctx->device));
-  Slot &s = ctx->slots[0];
-  if (s.busy) return fail(ctx, KUQ_E_STATE, "slot 0 still has an unread batch");
-  rc = ensure_ready(ctx);
+  int rc = begin_batch(ctx, 0, n_pieces, host_bases(piece_offsets, n_pieces), 0, false);
+  if (!rc) rc = ensure_ready(ctx);
   if (rc) return rc;
-  if (n_pieces > ctx->cfg.max_reads_per_batch) return fail(ctx, KUQ_E_CAPACITY, "%u pieces > slot capacity %u", n_pieces, ctx->cfg.max_reads_per_batch);
+  Slot &s = ctx->slots[0];
   if (ctx->bin_lo != 0 || ctx->rec_base != 0) return fail(ctx, KUQ_E_STATE, "set_lcas needs the whole database staged");
   for (uint32_t i = 0; i < n_pieces; i++) {
     // the reference skips sequences whose taxid the taxonomy does not hold (set_lcas.cpp:336-341): the caller's job
@@ -2567,14 +2536,12 @@ int kuq_set_lcas_batch(kuq_ctx *ctx, const char *bases, const uint64_t *piece_of
     for (uint32_t i = 0; i < n_pieces; i++) { c1 |= taxid[i] == 32630u; c2 |= taxid[i] == 81077u; }
     if (c1 && c2) return fail(ctx, KUQ_E_INVALID_ARG, "with KUQ_LCA_FORCE_CONTAMINANT a batch may hold pieces of taxid 32630 or of 81077, not both");
   }
-  uint64_t total = 0;
-  rc = upload_reads(ctx, s, bases, piece_offsets, n_pieces, &total);
+  rc = upload_reads(ctx, s, bases, piece_offsets);
   if (rc) return rc;
-  s.n_reads = n_pieces; s.flags = 0; s.total_bases = total; s.external = false;
   if (n_pieces) CU(cudaMemcpyAsync(s.d_unit, s.h_unit, n_pieces * 4ull, cudaMemcpyHostToDevice, s.stream));
   Params p;
   fill_params(ctx, s, p, s.d_bases, s.d_offsets, s.d_unit, n_pieces, 0);
-  p.lca_flags = flags & 3u;
+  p.lca_flags = flags & (KUQ_LCA_FORCE_CONTAMINANT | KUQ_LCA_RESET);
   {
     auto c1 = ctx->dense_of_raw.find(32630u), c2 = ctx->dense_of_raw.find(81077u);   // set_lcas.cpp:88-89
     p.lca_keep[0] = c1 == ctx->dense_of_raw.end() ? 0 : c1->second;

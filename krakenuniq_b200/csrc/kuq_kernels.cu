@@ -389,24 +389,24 @@ __global__ void __launch_bounds__(CTA_THREADS, 4) k_scan(const __grid_constant__
 // lookups belong to one range of a sharded database — the HLL insert of ReadCounts::add_kmer (classify.cpp:939).
 // Threads of a warp hold consecutive windows of a read: windows that share a minimizer read the same index
 // sector and the same pivots, which the load unit coalesces.
-// LEAN = the launch uses none of: probe statistics (flag 8), stored-zero marking (16), shard counting (32), hits-only
+// LEAN = the launch uses none of: probe statistics (KUQ_F_STATS), F_FOUND_ZERO, F_SHARD_COUNTING, hits-only
 // output, peer buffers.  Those are launch-uniform run-time switches; compiled out, the common path of the fused kernel
 // is a third shorter and measurably faster (profiles/layout_probe_r02.log: the search alone 1.87 -> 1.62 ms).
 template <int MODE, bool LEAN>
 __global__ void __launch_bounds__(256, 8) k_lookup(const __grid_constant__ Params p) {
   const DbView &db = p.db;
-  const uint32_t flags = LEAN ? (p.flags & 4u) : p.flags;
+  const uint32_t flags = LEAN ? (p.flags & KUQ_F_NO_COUNTS) : p.flags;
   const uint32_t only_hits = LEAN ? 0u : p.only_hits;
   const uint32_t n_peers = LEAN ? 0u : p.n_peers;
   const uint32_t hi_mask = (uint32_t)(db.key_mask >> 32);
-  const bool counting = (MODE == MODE_FUSED) && !(flags & 4u);
+  const bool counting = (MODE == MODE_FUSED) && !(flags & KUQ_F_NO_COUNTS);
   // hits of the fused path reach the sparse tier through the record flag (see below); dense-only / exact runs have
   // no sparse tier
-  // flag 32 (database sharded over GPUs, one database): the GPU that FINDS a hit owns its sketch work — register
-  // update and record flag happen in the lookup half, and the resolve half (on the GPU that owns the read) only adds
-  // the misses (taxon 0).  Valid because every looked-up window is counted exactly once in that layout.
-  const bool shard_counting = (flags & 32u) != 0;
-  const bool mark_seen = (counting || (MODE == MODE_LOOKUP && shard_counting)) && p.hll_mode <= 1u;
+  // F_SHARD_COUNTING (database sharded over GPUs, one database): the GPU that FINDS a hit owns its sketch work —
+  // register update and record flag happen in the lookup half, and the resolve half (on the GPU that owns the read)
+  // only adds the misses (taxon 0).  Valid because every looked-up window is counted exactly once in that layout.
+  const bool shard_counting = (flags & F_SHARD_COUNTING) != 0;
+  const bool mark_seen = (counting || (MODE == MODE_LOOKUP && shard_counting)) && p.hll_mode <= KUQ_HLL_CHUNKED;
   // only the text of this call's reads (the scratch beyond it may hold windows of an earlier call on the slot)
   const uint64_t g_begin = p.offsets[0], g_end = p.offsets[p.n_reads];
   // the scratch of the NEXT position of this thread is fetched while the current window is searched: the grid-stride
@@ -433,7 +433,7 @@ __global__ void __launch_bounds__(256, 8) k_lookup(const __grid_constant__ Param
       const uint64_t o0 = __ldg(o), o1 = __ldg(o + 1);
       uint64_t lo = o0 - db.rec_base;
       uint32_t n = (uint32_t)(o1 - o0);
-      if (flags & 8u) {   // measurement aid: algorithmic probe count of SURVEY.md §8(d)
+      if (flags & KUQ_F_STATS) {   // measurement aid: algorithmic probe count of SURVEY.md §8(d)
         atomicAdd(p.stats, 1ull);
         atomicAdd(p.stats + 1, (unsigned long long)(n ? 32 - __clz(n) : 0));
       }
@@ -463,7 +463,7 @@ __global__ void __launch_bounds__(256, 8) k_lookup(const __grid_constant__ Param
           const uint32_t hiw = __ldg(b + 3 * t + 1);
           if ((hiw & hi_mask) == chi) {
             taxon = __ldg(b + 3 * t + 2);                        // value = dense id
-            if (MODE == MODE_LOOKUP && taxon == 0 && (flags & 16u)) taxon = FOUND_ZERO;
+            if (MODE == MODE_LOOKUP && taxon == 0 && (flags & F_FOUND_ZERO)) taxon = FOUND_ZERO;
             // Sparse HLL tier of a hit (hyperloglogplus.cpp:499-512): the (taxon, encoded hash) pair is a function
             // of the RECORD, so instead of probing a hash set per window the record itself is flagged in the free
             // top bit of its key word — the sector is in L1/L2 already, the flag costs no DRAM read, and only the
@@ -476,7 +476,7 @@ __global__ void __launch_bounds__(256, 8) k_lookup(const __grid_constant__ Param
           }
         }
       }
-    } else if (flags & 8u) {
+    } else if (flags & KUQ_F_STATS) {
       atomicAdd(p.stats + 3, 1ull);                          // a window of another range: nothing fetched here
     }
     // only_hits: several DB ranges (GPUs) write their hits into one zero-initialised buffer, possibly over
@@ -493,11 +493,11 @@ __global__ void __launch_bounds__(256, 8) k_lookup(const __grid_constant__ Param
     }
     if (MODE == MODE_LOOKUP && shard_counting) {
       if (taxon != 0 && taxon != FOUND_ZERO) hll_update(p.regs, taxon, fmix64(canon));
-    } else if ((counting || (MODE == MODE_RESOLVE && !(flags & 4u))) && !(MODE == MODE_RESOLVE && shard_counting && taxon != 0)) {
+    } else if ((counting || (MODE == MODE_RESOLVE && !(flags & KUQ_F_NO_COUNTS))) && !(MODE == MODE_RESOLVE && shard_counting && taxon != 0)) {
       const uint64_t h = fmix64(canon);
       hll_update(p.regs, taxon, h);
       // direct set insert: misses (taxon 0 has no record to flag) and the resolve half, which only sees merged ids
-      if (p.hll_mode != 2u && !(mark_seen && taxon != 0) && !p.dense_flag[taxon]) {
+      if (p.hll_mode != KUQ_HLL_DENSE_ONLY && !(mark_seen && taxon != 0) && !p.dense_flag[taxon]) {
         const int ins = sparse_insert(p.sparse, taxon, encode_hash32(h));
         if (ins > 0) atomicAdd(p.sparse.distinct + taxon, 1u);
         else if (ins < 0) atomicExch(p.error_flag, 4u);       // set saturated
@@ -638,8 +638,8 @@ __global__ void __launch_bounds__(256, 4) k_resolve(const __grid_constant__ Para
   __shared__ uint2 s_runs[CTA_WARPS][RUN_BUF];
   const uint32_t lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const uint32_t warps_total = gridDim.x * CTA_WARPS;
-  const bool counting = !(p.flags & 4u);
-  const bool want_runs = !(p.flags & 2u);
+  const bool counting = !(p.flags & KUQ_F_NO_COUNTS);
+  const bool want_runs = !(p.flags & KUQ_F_NO_RUNS);
   const uint32_t *codes_src = p.codes_dense;
   // Same-address atomics serialise in L2 (about one per few cycles): a million reads per batch must not each hit
   // the run cursor, n_kmers[0] and n_reads[0].  Each warp therefore allocates run slots in blocks of RUN_BLOCK
@@ -647,7 +647,7 @@ __global__ void __launch_bounds__(256, 4) k_resolve(const __grid_constant__ Para
   uint32_t blk_next = 0, blk_end = 0;                           // this warp's block of run slots
   uint32_t acc_miss = 0, acc_unclassified = 0, acc_classified = 0;
   uint32_t unit_cur = 0xFFFFFFFFu, unit_miss = 0;               // misses of the current work unit, not yet booked
-  const bool units = counting && p.hll_mode == 0u && p.unit_id;
+  const bool units = counting && p.hll_mode == KUQ_HLL_PRELOAD && p.unit_id;
   const uint32_t unit_row0 = units ? p.unit_id[0] : 0u;
   auto book_unit = [&](uint32_t unit, uint32_t taxon, uint32_t cnt) {          // N(unit, taxon) += cnt
     const uint32_t row = unit - unit_row0;
@@ -672,7 +672,7 @@ __global__ void __launch_bounds__(256, 4) k_resolve(const __grid_constant__ Para
   // that do not depend on the read's outcome are therefore issued one read ahead: while read r is resolved, the
   // codes of read r+1 (first PRE_SLOTS x 32 windows) and the offset / window count / unit of read r+2 are in flight.
   constexpr int PRE_SLOTS = 4;
-  const bool want_codes = (p.flags & 1u) != 0;
+  const bool want_codes = (p.flags & KUQ_F_WANT_CODES) != 0;
   uint64_t base_a = 0, base_b = 0;                              // read r, read r+1
   uint32_t nwin_a = 0, nwin_b = 0, unit_a = 0, unit_b = 0;
   uint32_t pre[PRE_SLOTS];
@@ -1222,7 +1222,7 @@ int classify_smem_bytes() { return N_STAGES * STAGE_BYTES + (int)sizeof(SharedSt
 // picks the lean instantiation when the launch uses none of the rare switches (see k_lookup)
 template <int MODE>
 static void launch_lookup(const Params &q, int lgrid, cudaStream_t stream) {
-  const bool lean = !(q.flags & (8u | 16u | 32u)) && !q.only_hits && !q.n_peers;
+  const bool lean = !(q.flags & (KUQ_F_STATS | F_FOUND_ZERO | F_SHARD_COUNTING)) && !q.only_hits && !q.n_peers;
   if (lean) k_lookup<MODE, true><<<lgrid, 256, 0, stream>>>(q);
   else k_lookup<MODE, false><<<lgrid, 256, 0, stream>>>(q);
 }
@@ -1240,23 +1240,23 @@ int launch_classify(int mode, const Params &p, int n_sm, cudaStream_t stream, cu
   if (stage_events) cudaEventRecord(stage_events[0], stream);
   const int lgrid = (int)min((uint64_t)n_sm * 8 * 8, (p.total_bases + 255) / 256);
   const bool quick = p.quick_min != 0 && mode != MODE_LOOKUP;
-  const bool exact = p.hll_mode == 3u && mode != MODE_LOOKUP;
+  const bool exact = p.hll_mode == KUQ_HLL_EXACT && mode != MODE_LOOKUP;
   if (exact) {
     // classifyExact: plain lookup (no sketch work), then the k-mer sets, then the usual resolve
     Params q = p;
     if (mode == MODE_FUSED) {
-      q.only_hits = 0; q.n_peers = 0; q.flags &= ~16u;
+      q.only_hits = 0; q.n_peers = 0; q.flags &= ~F_FOUND_ZERO;
       launch_lookup<MODE_LOOKUP>(q, lgrid, stream);
     } else {
-      q.flags |= 4u;                                         // merged codes → codes_dense, no sketches
+      q.flags |= KUQ_F_NO_COUNTS;                                     // merged codes → codes_dense, no sketches
       launch_lookup<MODE_RESOLVE>(q, lgrid, stream);
     }
-    if (!(p.flags & 4u)) { k_exact_insert<<<lgrid, 256, 0, stream>>>(p); launches++; }
+    if (!(p.flags & KUQ_F_NO_COUNTS)) { k_exact_insert<<<lgrid, 256, 0, stream>>>(p); launches++; }
   } else if (quick && p.quick_stop) {
     // lookup first, end every read at its quick_min-th hit, then count what is left
     Params q = p;
     if (mode == MODE_FUSED) {
-      q.only_hits = 0; q.n_peers = 0; q.flags &= ~16u;
+      q.only_hits = 0; q.n_peers = 0; q.flags &= ~F_FOUND_ZERO;
       launch_lookup<MODE_LOOKUP>(q, lgrid, stream);
       launches++;
       q.codes_in = p.codes_dense;
@@ -1318,8 +1318,8 @@ __global__ void __launch_bounds__(256) k_set_lcas(const __grid_constant__ Params
       uint32_t old = *reinterpret_cast<volatile uint32_t *>(val);
       for (;;) {
         uint32_t nw;
-        if (p.lca_flags & 2u) nw = 0;                                     // -R, :458-459
-        else if (!(p.lca_flags & 1u)) nw = lca_dense(p.tax, t, old);      // :461
+        if (p.lca_flags & KUQ_LCA_RESET) nw = 0;                                           // -R, :458-459
+        else if (!(p.lca_flags & KUQ_LCA_FORCE_CONTAMINANT)) nw = lca_dense(p.tax, t, old);  // :461
         else if (old != 0 && (old == p.lca_keep[0] || old == p.lca_keep[1])) nw = old;   // -T: contaminants stick, :465-466
         else if (t == p.lca_keep[0] || t == p.lca_keep[1]) nw = t;        // :467-470
         else nw = lca_dense(p.tax, t, old);                               // :472

@@ -25,12 +25,18 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
-struct kuq_layout_result;
+#include "../../include/kuq.h"
 
 namespace kuq {
 
+// Params::flags holds the public KUQ_F_* bits of kuq.h and two internal bits the library sets above them:
+constexpr uint32_t F_FOUND_ZERO = 16u;        // MODE_LOOKUP reports a stored taxon 0 as FOUND_ZERO (kuq_mark_zero_hits)
+constexpr uint32_t F_SHARD_COUNTING = 32u;    // the lookup half does the sketch work of its hits (kuq_set_shard_counting)
+static_assert(F_FOUND_ZERO > (KUQ_F_WANT_CODES | KUQ_F_NO_RUNS | KUQ_F_NO_COUNTS | KUQ_F_STATS),
+              "the internal launch flags must not overlap the public KUQ_F_* bits");
+
 constexpr uint32_t AMBIG = 0xFFFFFFFFu;
-// MODE_LOOKUP with flag 16: the key IS in the database but stores taxon 0 (an un-LCA'd record).  With several
+// MODE_LOOKUP with F_FOUND_ZERO: the key IS in the database but stores taxon 0 (an un-LCA'd record).  With several
 // databases that still ends the search (classify.cpp:928-936), so the lookup has to tell it from a miss.
 constexpr uint32_t FOUND_ZERO = 0xFFFFFFFDu;
 constexpr int CTA_THREADS = 256;
@@ -122,7 +128,7 @@ struct Params {
   // outputs
   uint32_t *call;               // [n_reads] taxid
   uint32_t *n_windows;          // [n_reads]
-  uint32_t *codes;              // per window, indexed like bases (taxids; only with flag 1)
+  uint32_t *codes;              // per window, indexed like bases (taxids; only with KUQ_F_WANT_CODES)
   uint64_t total_bases;
   // scratch between the stages (indexed like bases)
   uint64_t *canon;              // canonical k-mer of the window
@@ -143,7 +149,7 @@ struct Params {
   uint32_t n_peers;
   uint32_t *peer_codes[8];
   uint64_t peer_bounds[9];
-  unsigned long long *stats;    // flag 8: [0] += looked-up windows, [1] += sum of ceil(log2(bin size + 1))
+  unsigned long long *stats;    // KUQ_F_STATS: [0] += looked-up windows, [1] += sum of ceil(log2(bin size + 1))
   // per-taxon state
   uint8_t *regs;                // [n_sketch][4096]
   unsigned long long *n_kmers;  // [n_sketch]
